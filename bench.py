@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- paired reads/s of the `kallisto quant` hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE config 2 -- a human-GENCODE-v44-like transcriptome index
 (built by the unmodified reference `kallisto index`, k=31; synthetic stand-in, see benchdata.py)
@@ -15,10 +15,15 @@ table is finalised and the EM is run ONCE, inside the timed region (it is part o
            host-buffer figure of the C ABI is listed under config.pinned_host_buffers;
   roofline  = match_kernel: algorithmic bytes (SURVEY.md 8d / DESIGN.md) / CUDA-event time, vs
            MEASURED_PEAKS.json hbm_gbs;
-  --impl reference = oracle/_ref/kallisto (the unmodified reference, built from /root/reference by
+  --impl reference = oracle/_ref/kallisto (the unmodified reference, built from its sources by
            oracle/Makefile) `quant -t <best>` on the SAME FASTQ files (all K x P pairs of rank 0's job, one
            run, process wall clock); cpu_baseline = that run when it happened on this box, else a 2 M-pair sample.
+  --dump-outputs DIR = what the reported timed job returned to its caller, as DIR/<name>.npy (float64): est_counts,
+           eff_lens, em_rounds, the fragment-length histogram and the EC table (counts, set sizes, transcript ids;
+           arrays longer than 2^20 are replaced by a fixed seeded sample of 2^20 entries, < 64 MB in all).  The inputs
+           are pure functions of the arguments, so two builds can be compared output for output.
 Every step uses different reads and each batch (pairs_per_step x 200 B) is larger than L2.
+The index, the transcriptome and the FASTQ files are cached in temporary directories, never in the source tree.
 """
 import argparse
 import json
@@ -36,7 +41,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 import benchdata  # noqa: E402
 
-DATA = os.path.join(ROOT, "bench_data")
+DATA = os.path.join(tempfile.gettempdir(), "kallisto_b200_bench_data_%d" % os.getuid())
 READ_LEN = 100
 
 
@@ -45,7 +50,7 @@ def log(*a):
 
 
 # ---------------------------------------------------------------------------------------------
-# workload: index + transcriptome (cached under bench_data/, rebuilt with the reference if absent)
+# workload: index + transcriptome (cached under DATA, rebuilt with the reference if absent)
 # ---------------------------------------------------------------------------------------------
 def workload(genes):
     import fcntl
@@ -71,7 +76,7 @@ def workload(genes):
 def _build_workload(genes, idx, txf):
     if not (os.path.exists(idx) and os.path.exists(txf)):
         from oracle import oracle as O
-        log("building workload for %d genes (one-off, cached in bench_data/)" % genes)
+        log("building workload for %d genes (one-off, cached in %s)" % (genes, DATA))
         t0 = time.time()
         tx = benchdata.make_transcriptome(genes, seed=44)
         codes = np.zeros(256, np.uint8)
@@ -83,12 +88,12 @@ def _build_workload(genes, idx, txf):
         packed = (c[:, 0] | (c[:, 1] << 2) | (c[:, 2] << 4) | (c[:, 3] << 6)).astype(np.uint8)
         np.savez(txf + ".tmp.npz", packed=packed, lens=tx.lens)
         os.replace(txf + ".tmp.npz", txf)
-        if not os.path.exists(idx):
-            O.build()
+        if not os.path.exists(idx):     # oracle/_ref/kallisto is built by __graft_entry__.build(), not here: the tree may be read-only
             with tempfile.TemporaryDirectory(dir=DATA) as td:
                 fa = os.path.join(td, "tx.fa")
                 tx.write_fasta(fa)
-                O.ref_run(["index", "-t", str(min(32, os.cpu_count() or 8)), "-i", idx + ".tmp", fa])
+                # -T: the reference's scratch directory defaults to ./tmp, and the working directory may be read-only
+                O.ref_run(["index", "-t", str(min(32, os.cpu_count() or 8)), "-T", os.path.join(td, "tmp"), "-i", idx + ".tmp", fa])
             os.replace(idx + ".tmp", idx)
         log("workload built in %.0f s" % (time.time() - t0))
 
@@ -309,6 +314,23 @@ def reference_sample(idx, files, repeats=1):
                 t_total=round(dt, 2))
 
 
+DUMP_MAX_ELEMS = 1 << 20
+
+
+def dump_outputs(d, em, ec_table, flens):
+    """The arrays the timed job handed to its caller, as float64 .npy files (7 arrays of at most 2^20 entries)."""
+    eo, et, ec, _ = ec_table
+    out = {"est_counts": em["est_counts"], "eff_lens": em["eff_lens"], "em_rounds": np.array([em["rounds"]]),
+           "fragment_lengths": flens, "ec_counts": ec, "ec_sizes": np.diff(eo.astype(np.int64)), "ec_tids": et}
+    os.makedirs(d, exist_ok=True)
+    for name, a in out.items():
+        a = np.asarray(a, np.float64)
+        if len(a) > DUMP_MAX_ELEMS:     # fixed seed: the same positions for arrays of the same length
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), DUMP_MAX_ELEMS, replace=False))]
+        np.save(os.path.join(d, name + ".npy"), a)
+    log("outputs of the timed job written to %s" % d)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -319,6 +341,7 @@ def main():
     ap.add_argument("--genes", type=int, default=int(os.environ.get("KB_BENCH_GENES", "62000")))
     ap.add_argument("--pairs-per-step", type=int, default=int(os.environ.get("KB_BENCH_PAIRS", "2000000")))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the reported timed job to DIR/<name>.npy")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -467,6 +490,8 @@ def main():
         eo, et, ec, _ = mc.ec_table()
         ln = np.diff(eo.astype(np.int64))
         em_shape = {"n_ecs": int(len(ln)), "n_multi_ecs": int((ln > 1).sum()), "nnz_multi": int(ln[ln > 1].sum())}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, em, (eo, et, ec, None), mc.flens)
     mc.close()
 
     # ---- pinned host buffers through the C ABI, H2D inside (host wall clock) ----

@@ -234,7 +234,8 @@ def ref_run(args, cwd=None, check=True):
 
 
 def ref_index(fasta, out, k=31, threads=1):
-    ref_run(["index", "-i", out, "-k", str(k), "-t", str(threads), fasta])
+    # -T: the reference's scratch directory defaults to ./tmp, and the working directory may be read-only
+    ref_run(["index", "-T", out + ".scratch", "-i", out, "-k", str(k), "-t", str(threads), fasta])
     return out
 
 

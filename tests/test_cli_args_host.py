@@ -1,8 +1,11 @@
 """CPU: option validation of the kallisto_b200 command line against the unmodified reference binary
 (CheckOptionsEM / CheckOptionsBus, src/main.cpp:1283-1805): same exit code and the same `Error:` lines for
-invocations that are rejected before any device work.  Skipped where oracle/_ref/kallisto is not built."""
+invocations that are rejected before any device work.  The reference's answers are stored in
+tests/golden/cli_errors.json (`python -m tests.test_cli_args_host` rewrites it with oracle/_ref/kallisto)."""
+import json
 import os
 import subprocess
+import sys
 
 import pytest
 
@@ -10,7 +13,8 @@ from oracle import oracle as O
 from tests import util
 
 BIN = os.path.join(util.ROOT, "kallisto_b200", "kallisto_b200")
-pytestmark = pytest.mark.skipif(not (O.have_ref() and os.path.exists(BIN)), reason="needs oracle/_ref/kallisto and the CLI")
+GOLDEN_ERRORS = os.path.join(util.GOLDEN, "cli_errors.json")
+pytestmark = pytest.mark.skipif(not os.path.exists(BIN), reason="needs the kallisto_b200 CLI")
 
 D = os.path.join(util.GOLDEN, "config1")
 IDX, R1, R2 = (os.path.join(D, f) for f in ("transcripts.kidx", "reads_1.fastq.gz", "reads_2.fastq.gz"))
@@ -60,11 +64,32 @@ def errors(binary, args, cwd):
     return r.returncode, [l.strip() for l in r.stderr.splitlines() if l.startswith("Error")]
 
 
+def case_key(args):
+    return " ".join(os.path.relpath(x, util.ROOT) if os.path.isabs(x) else x for x in args)
+
+
+def reference_errors():
+    with open(GOLDEN_ERRORS) as f:
+        return {c["args"]: (c["exit_code"], c["errors"]) for c in json.load(f)}
+
+
 @pytest.mark.parametrize("args", CASES, ids=lambda a: " ".join(os.path.basename(x) for x in a)[:60])
 def test_rejected_like_the_reference(args, tmp_path):
-    (tmp_path / "a").mkdir()
-    (tmp_path / "b").mkdir()
-    want = errors(O.REF_BIN, args, str(tmp_path / "a"))
-    got = errors(BIN, args, str(tmp_path / "b"))
+    want = reference_errors()[case_key(args)]
+    got = errors(BIN, args, str(tmp_path))
     assert want[0] != 0, "the reference accepts this invocation: not a validation case"
     assert got == want
+
+
+if __name__ == "__main__":
+    # rewrite the fixture from the unmodified reference binary
+    import tempfile
+    out = []
+    for args in CASES:
+        with tempfile.TemporaryDirectory() as td:
+            rc, lines = errors(O.REF_BIN, args, td)
+        out.append({"args": case_key(args), "exit_code": rc, "errors": lines})
+    with open(GOLDEN_ERRORS, "w") as f:
+        json.dump(out, f, indent=1)
+        f.write("\n")
+    sys.exit(0)

@@ -1,6 +1,6 @@
 """GPU: the CUDA path against the oracle on the random transcriptomes of tests/test_oracle_fuzz.py (other k, reads
 barely longer than k, Ns, unrelated reads, all strand modes).  The oracle itself is pinned on the unmodified
-reference for exactly these inputs by the CPU test; here the reference binary is only needed to build the index."""
+reference for exactly these inputs by the CPU test; the indices are the reference's, stored in tests/golden/fuzz."""
 import numpy as np
 import pytest
 
@@ -9,7 +9,7 @@ from oracle import oracle as O
 from tests import util
 from tests.test_oracle_fuzz import make_case
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref/kallisto not built")]
+pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.parametrize("seed,k,read_len", [(1, 31, 75), (2, 21, 50), (3, 15, 36), (4, 31, 33), (5, 27, 150)])

@@ -12,7 +12,7 @@ from tests.test_oracle_bus_fuzz import layout
 from tests.test_oracle_bus_paired import sorted_records
 from tests.test_oracle_fuzz import make_case
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not O.have_ref(), reason="the random indices are built by oracle/_ref/kallisto")]
+pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.parametrize("seed", range(8))

@@ -2,18 +2,29 @@
 reference binary on random small transcriptomes with random technology layouts: barcode / UMI pieces anywhere in the
 files, with and without a UMI, one sequence read or a pair with random start offsets, tag sequences of several lengths
 (short ones must match exactly, src/ProcessReads.cpp:1517), strand modes, --num, reads that are too short for their
-slices, Ns in barcodes, UMIs and tags.  Skipped where oracle/_ref/kallisto is not present."""
+slices, Ns in barcodes, UMIs and tags.  The reference's results are stored in tests/golden/fuzz/ref_bus.npz (record
+count and SHA-256 of the sorted records, EC sets, fragment lengths; `python -m tests.test_oracle_bus_fuzz` rewrites it
+with oracle/_ref/kallisto after `python -m tests.test_oracle_fuzz` has stored the indices)."""
+import hashlib
 import os
 import subprocess
+import sys
 
 import numpy as np
 import pytest
 
 from oracle import oracle as O
 from tests.test_oracle_bus_paired import sorted_records
-from tests.test_oracle_fuzz import make_case
+from tests.test_oracle_fuzz import FUZZ, make_case
 
-pytestmark = pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref/kallisto not built")
+SEEDS = range(16)
+KS = [31, 21, 15, 27]
+INDEX_CASES = [(50 + seed, KS[seed % 4], KS[seed % 4] + 2) for seed in SEEDS]     # (seed, k, read length) of make_case
+REF_RESULTS = os.path.join(FUZZ, "ref_bus.npz")
+
+
+def records_digest(rec):
+    return hashlib.sha256(sorted_records(rec.copy()).tobytes()).hexdigest()
 
 
 def layout(rng, paired, tag, no_umi):
@@ -47,15 +58,15 @@ def tech_string(bc, umi_user, seq, seq2):
     return "%s:%s:%s" % (t(bc), t(umi_user) if umi_user else "-1,-1,-1", t(s))
 
 
-@pytest.mark.parametrize("seed", range(16))
-def test_random_layout(seed, tmp_path):
+def bus_case(seed, tmp_path):
+    """Inputs of one random layout: -> dict(index, files as lists of sequences, their paths, layout, reference arguments)."""
     rng = np.random.default_rng(1000 + seed)
     paired = bool(seed & 1)
     tag = [None, None, b"ACGTTGCA", b"TTGCA", b"ATTGCGCAATG"][seed % 5]
     no_umi = tag is None and seed % 3 == 0
     strand = int(rng.integers(0, 3))
     num = bool(rng.random() < 0.3)
-    k = [31, 21, 15, 27][seed % 4]
+    k = KS[seed % 4]
     idx, r1, r2, _ = make_case(str(tmp_path), 50 + seed, k, int(rng.integers(k + 2, 90)), 1200)
     bc, umi_user, seq, seq2, nfiles, pre = layout(rng, paired, tag, no_umi)
     lut = np.frombuffer(b"ACGT", np.uint8)
@@ -109,17 +120,50 @@ def test_random_layout(seed, tmp_path):
         args.append("--num")
     if tag:
         args += ["--tag", tag.decode()]
-    r = subprocess.run([O.REF_BIN] + args + paths, capture_output=True, text=True)
+    return dict(idx=idx, files=files, paths=paths, args=args, bc=bc, umi_user=umi_user, seq=seq, seq2=seq2, strand=strand,
+                num=num, tag=tag, paired=paired)
+
+
+def reference_bus(c, out):
+    """-> {name: array}: the reference's record count and records digest, EC sets and fragment lengths."""
+    r = subprocess.run([O.REF_BIN] + c["args"] + c["paths"], capture_output=True, text=True)
     assert r.returncode in (0, 1), r.stderr[-500:]          # 1: nothing pseudoaligned
-    hdr, ref = O.read_bus(str(tmp_path / "o" / "output.bus"))
+    hdr, ref = O.read_bus(os.path.join(out, "output.bus"))
+    ecs = O.read_matrix_ec(os.path.join(out, "matrix.ec")) if len(ref) else []
+    res = {"n_records": np.array(len(ref)), "records_sha256": np.array(records_digest(ref)),
+           "ec_offsets": np.cumsum([0] + [len(e) for e in ecs]), "ec_tids": np.array([t for e in ecs for t in e], np.int64)}
+    if c["paired"]:
+        res["flens"] = np.array(open(os.path.join(out, "flens.txt")).read().split(), np.uint32)
+    return res
+
+
+@pytest.mark.parametrize("seed", SEEDS)
+def test_random_layout(seed, tmp_path):
+    c = bus_case(seed, tmp_path)
+    with np.load(REF_RESULTS) as z:
+        ref = {name[len("seed%d_" % seed):]: z[name] for name in z.files if name.startswith("seed%d_" % seed)}
+    tag, umi_user = c["tag"], c["umi_user"]
     taglen = len(tag) if tag else 0
     umi = None if umi_user is None else [(umi_user[0][0], umi_user[0][1] + taglen, umi_user[0][2])]
-    ix = O.OracleIndex(idx)
-    m = O.bus_model(ix, files, bc, umi, seq, seq2, strand=strand, num=num, tag=tag)
-    assert len(m["records"]) == len(ref), (args, len(m["records"]), len(ref))
-    assert sorted_records(m["records"]).tobytes() == sorted_records(ref.copy()).tobytes(), args
-    ref_ecs = O.read_matrix_ec(str(tmp_path / "o" / "matrix.ec")) if len(ref) else []
-    assert m["ecs"] == ref_ecs
-    if paired:
-        fl = np.array(open(tmp_path / "o" / "flens.txt").read().split(), np.uint32)
-        np.testing.assert_array_equal(m["flens"][0], fl)
+    ix = O.OracleIndex(c["idx"])
+    m = O.bus_model(ix, c["files"], c["bc"], umi, c["seq"], c["seq2"], strand=c["strand"], num=c["num"], tag=tag)
+    assert len(m["records"]) == int(ref["n_records"]), (c["args"], len(m["records"]), int(ref["n_records"]))
+    assert records_digest(m["records"]) == str(ref["records_sha256"]), c["args"]
+    offs, tids = ref["ec_offsets"], ref["ec_tids"]
+    assert m["ecs"] == [tuple(int(t) for t in tids[offs[i]:offs[i + 1]]) for i in range(len(offs) - 1)]
+    if c["paired"]:
+        np.testing.assert_array_equal(m["flens"][0], ref["flens"])
+
+
+if __name__ == "__main__":
+    # rewrite tests/golden/fuzz/ref_bus.npz from the unmodified reference binary
+    import pathlib
+    import tempfile
+    results = {}
+    for seed in SEEDS:
+        with tempfile.TemporaryDirectory() as td:
+            c = bus_case(seed, pathlib.Path(td))
+            for name, a in reference_bus(c, os.path.join(td, "o")).items():
+                results["seed%d_%s" % (seed, name)] = a
+    np.savez_compressed(REF_RESULTS, **results)
+    sys.exit(0)

@@ -2,7 +2,7 @@
 # Phase detail of the command line on the benchmark's FASTQ files (bench.py writes them to /dev/shm/kb_bench_cache):
 # KB_CLI_TIMING=2 prints every phase and round; `strace -c`-free, just wall clocks.  Usage: tools/cli_detail.sh [devices]
 D=$(ls -d /dev/shm/kb_bench_cache/g62000_p2000000_k*_L100 | head -1)
-IDX=bench_data/g62000.kidx
+IDX=$(python -c 'import bench; print(bench.DATA)')/g62000.kidx
 DEV=${1:-0}
 for i in 1 2 ${KB_DETAIL_REPS:-3}; do
   S=$(date +%s%N)

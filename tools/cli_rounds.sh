@@ -3,7 +3,7 @@
 # kb_pseudoalign_batch_pe (offset scan + H2D copies, waits for the copy) and the wall clock; the rest of a round is
 # waiting for the parser.  Needs the benchmark's FASTQ files (bench.py / tools/parse_sweep.sh write them).
 D=$(ls -d /dev/shm/kb_bench_cache/g62000_p2000000_k20_w5_L100 | head -1)
-KB_CLI_TIMING=2 kallisto_b200/kallisto_b200 quant -i bench_data/g62000.kidx -o $D/rounds_out --plaintext -t 64 --device 0 $D/r_1.fq $D/r_2.fq 2>&1 | grep -a "timing" > /tmp/rounds.log
+KB_CLI_TIMING=2 kallisto_b200/kallisto_b200 quant -i $(python -c 'import bench; print(bench.DATA)')/g62000.kidx -o $D/rounds_out --plaintext -t 64 --device 0 $D/r_1.fq $D/r_2.fq 2>&1 | grep -a "timing" > /tmp/rounds.log
 python3 - <<'PY'
 import re
 calls=[]; ats=[]

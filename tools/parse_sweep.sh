@@ -9,7 +9,7 @@ idx, concat, lens = bench.workload(62000)
 bench.fastq_job_files(62000, 2000000, 20, 5, lambda: benchdata.TorchSimulator(concat, lens, "cuda:0", read_len=100))
 PY
 D=$(ls -d /dev/shm/kb_bench_cache/g62000_p2000000_k20_w5_L100 | head -1)
-IDX=bench_data/g62000.kidx
+IDX=$(python -c 'import bench; print(bench.DATA)')/g62000.kidx
 python - <<'PY' &
 import torch, time
 torch.zeros(1, device="cuda")      # keeps the GPU initialised, as the benchmark's parent process does
